@@ -19,6 +19,8 @@ Rank 0 prints ONE JSON line.  Extra objects (see DESIGN.md "Measurement"):
 the bench configuration itself, >= 3 timed iterations within --ref-budget-s; --ref-cuda sets its device.cuda = True;
 --ref-cross-check adds the oracle CPU port (oracle/runner.py) as a cross-check.  --scaling strong splits the workload's
 n_rollout_threads over the ranks instead of giving each rank all of them.
+--dump-outputs DIR writes what the last timed iteration computed as DIR/<name>.npy (see dump_outputs), so that two
+builds run with the same arguments -- hence the same seeded inputs -- can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -155,6 +157,43 @@ def timed_iterations(runner, steps, warmup, torch, dist_on, sample_clocks=False)
         torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
     runner._bench_episode = ep
     return ms.item(), launches, (sampler.summary() if sampler else None)
+
+
+DUMP_ROWS = 16384   # rollout rows (t, thread) of the seeded sample written per buffer tensor
+
+
+def dump_outputs(runner, out_dir, torch):
+    """Write what the runner's last iteration handed back (rank 0's shard): the train infos of every agent and of the
+    critic (float64), the flat parameters of every actor and of the critic after the update, the ValueNorm statistics,
+    and a fixed, seeded sample of DUMP_ROWS rollout rows of the buffers it filled -- each agent's actions and their
+    log-probs, the critic's value predictions, returns and advantages (float32).  0.9 MB at C2."""
+    import numpy as np
+
+    torch.cuda.synchronize()
+    T, N = runner.algo_args["train"]["episode_length"], runner.n_local
+    pick = torch.randperm(T * N, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values.to(runner.device)
+
+    def rows(x):   # [T or T + 1, N, ...] -> the sampled rows of the first T steps
+        return x[:T].reshape(T * N, *x.shape[2:]).index_select(0, pick)
+
+    actor_infos, critic_info = runner.last_train_infos
+    out = {f"actor_info_{k}": np.array([info[k] for info in actor_infos], np.float64) for k in sorted(actor_infos[0])}
+    out.update({f"critic_info_{k}": np.array([critic_info[k]], np.float64) for k in sorted(critic_info)})
+    for a, (actor, buf) in enumerate(zip(runner.actor, runner.actor_buffer)):
+        out[f"actor{a}_params"] = actor.actor.params
+        out[f"actor{a}_actions"] = rows(buf.actions)
+        out[f"actor{a}_action_log_probs"] = rows(buf.action_log_probs)
+    cb = runner.critic_buffer
+    out["critic_params"] = runner.critic.critic.params
+    for name in ("value_preds", "returns", "advantages"):
+        out[f"critic_{name}"] = rows(getattr(cb, name))
+    if runner.value_normalizer is not None:
+        out["value_normalizer"] = torch.cat([v.reshape(-1).double() for v in runner.value_normalizer.state_dict().values()])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        if torch.is_tensor(v):
+            v = v.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), v if v.dtype == np.float64 else v.astype(np.float32))
 
 
 def kernel_profile(runner, torch):
@@ -510,7 +549,13 @@ def main():
     ap.add_argument("--ref-cross-check", action="store_true", help="--impl reference: also time the oracle CPU port")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--profile-out", default="", help="write the per-kernel event profile of one iteration here")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed iteration computed to DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     # the contract is ONE JSON line on stdout: everything the runner / env print (the reference prints its spaces
     # and progress lines) goes to stderr
     # -- at the file-descriptor level, so that C libraries (NCCL prints its version banner to fd 1) are covered too
@@ -572,6 +617,8 @@ def main():
     NET_SHAPES.update(out=(sp.n if sp.__class__.__name__ == "Discrete" else sp.shape[0]), discrete=sp.__class__.__name__ == "Discrete",
                       avail=runner.actor_buffer[0].available_actions is not None)
     ms, launches, clocks = timed_iterations(runner, a.steps, a.warmup, torch, dist_on, sample_clocks=(rank == 0))
+    if a.dump_outputs and rank == 0:
+        dump_outputs(runner, a.dump_outputs, torch)
     n_global = wl["n"] * (1 if STRONG else world)
     value = T * n_global * a.steps / (ms / 1e3)
     line = dict(base, value=value, ms_per_step=ms / a.steps, gpu_launches=int(launches), clocks=clocks)

@@ -1,19 +1,14 @@
 """CPU: every on-policy tuned config of the reference (tuned_configs/*/*/{happo,hatrpo,haa2c,mappo}/config.json) is
 structurally inside the device path: its model section maps to an hb_net_desc the library lays out (host-only call),
 its algorithm is registered, and the one documented exception (share_param together with a recurrent policy) does not
-occur in any of them.  Skipped where the reference checkout is not available (e.g. on the GPU box)."""
+occur in any of them.  The configs are stored in tests/golden/reference_tuned_configs.json
+(tests/golden/make_reference_configs.py)."""
 import ctypes as C
-import glob
 import json
 import os
 
-import pytest
-
-REF = os.environ.get("HARL_REFERENCE", "/root/reference")
-FILES = sorted(glob.glob(os.path.join(REF, "tuned_configs", "*", "*", "*", "config.json")))
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_tuned_configs.json")
 ON_POLICY = ("happo", "hatrpo", "haa2c", "mappo")
-
-pytestmark = pytest.mark.skipif(not FILES, reason="reference tuned_configs not available")
 
 
 def test_on_policy_tuned_configs_are_in_scope():
@@ -22,9 +17,10 @@ def test_on_policy_tuned_configs_are_in_scope():
     from harl_b200.nets import make_desc
     from harl_b200.runners import RUNNER_REGISTRY
 
+    with open(GOLDEN, encoding="utf-8") as fh:
+        configs = json.load(fh)
     seen = 0
-    for f in FILES:
-        blob = json.load(open(f))
+    for f, blob in configs.items():
         algo = blob["main_args"]["algo"]
         if algo not in ON_POLICY:
             continue
