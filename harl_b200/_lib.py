@@ -208,7 +208,7 @@ for _name, (_res, _args) in SIGNATURES.items():
     _fn.argtypes = _args
 
 HB_ERR_UNSUPPORTED = -2
-GEMM_IMPLS = {"fp32": 0, "3xtf32": 1, "tf32": 2}
+GEMM_IMPLS = {"fp32": 0, "3xtf32": 1}
 if os.environ.get("HB_GEMM_IMPL"):
     lib.hb_set_gemm_impl(GEMM_IMPLS[os.environ["HB_GEMM_IMPL"]])
 _NO_CHECK = {"hb_version", "hb_last_error", "hb_workspace_bytes", "hb_trpo_workspace_bytes", "hb_kernel_launch_count", "hb_profile_end", "hb_get_gemm_impl", "hb_get_rnn_impl", "hb_get_trpo_jvp_impl", "hb_get_fused_update", "hb_get_gae_impl", "hb_comm_status"}

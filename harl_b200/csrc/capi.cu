@@ -18,13 +18,7 @@
 
 namespace hb {
 
-// Rows per kernel launch.  HB_CHUNK_ROWS overrides it for tuning runs (read once).
-static int64_t chunk_rows_init() {
-  const char* e = getenv("HB_CHUNK_ROWS");
-  long long v = e ? atoll(e) : 0;
-  return v >= 1024 ? (int64_t)v : (int64_t)1 << 20;
-}
-static const int64_t CHUNK_ROWS = chunk_rows_init();
+constexpr int64_t CHUNK_ROWS = (int64_t)1 << 20;   // rows per kernel launch
 
 struct Work {
   float* x0;
@@ -139,9 +133,8 @@ static int trunk_forward(const hb_net_desc* d, const PrepLayout& Q, const float*
   const float* x = w.x0;
   int ldx = Q.kpad[0];
   for (int l = 0; l < Q.n_layers; ++l) {
-    const int impl = gemm_impl();
-    if (impl != 0)
-      rc = launch_tc_linear_ln_fwd(impl == 1 ? 3 : 1, d->activation, x, ldx, prep + Q.tk[l], Q.tk_chunks[l],
+    if (gemm_impl() != 0)
+      rc = launch_tc_linear_ln_fwd(d->activation, x, ldx, prep + Q.tk[l], Q.tk_chunks[l],
                                    prep + Q.bias[l], prep + Q.lnw[l], prep + Q.lnb[l], w.Z[l], w.Y[l], w.stats[l], rows,
                                    Q.n[l], Q.kpad[l], st);
     else
@@ -162,16 +155,15 @@ static int trunk_backward(const hb_net_desc* d, const ParamLayout& P, const Prep
   float* dnext = w.dB;
   int rc = HB_OK;  // the LN + activation backward of the last block is fused into the head kernel (w.dA already holds dZ_L)
   const int impl = gemm_impl();
-  const int passes = impl == 1 ? 3 : 1;
   for (int l = L - 1; l >= 1; --l) {
     if (impl != 0)
-      rc = launch_tc_dw_accum(passes, dcur, Q.n[l], w.Y[l - 1], Q.n[l - 1], Q.k[l], w.dwpart + P.w[l], grad + P.b[l], rows,
+      rc = launch_tc_dw_accum(dcur, Q.n[l], w.Y[l - 1], Q.n[l - 1], Q.k[l], w.dwpart + P.w[l], grad + P.b[l], rows,
                               w.ptotal, st);
     else
       rc = launch_dw_accum(dcur, Q.n[l], w.Y[l - 1], Q.n[l - 1], Q.k[l], grad + P.w[l], grad + P.b[l], rows, st);
     if (rc) return rc;
     if (impl != 0)
-      rc = launch_tc_dx_ln_bwd(passes, d->activation, dcur, Q.n[l], prep + Q.tkt[l], Q.tkt_chunks[l], w.Z[l - 1],
+      rc = launch_tc_dx_ln_bwd(d->activation, dcur, Q.n[l], prep + Q.tkt[l], Q.tkt_chunks[l], w.Z[l - 1],
                                w.stats[l - 1], prep + Q.lnw[l - 1], dnext, grad + P.lnw[l - 1], grad + P.lnb[l - 1], rows,
                                Q.n[l - 1], w.dwpart - grad, w.ptotal, st);
     else
@@ -181,7 +173,7 @@ static int trunk_backward(const hb_net_desc* d, const ParamLayout& P, const Prep
     float* t = dcur; dcur = dnext; dnext = t;
   }
   if (impl != 0)
-    return launch_tc_dw_accum(passes, dcur, Q.n[0], w.x0, Q.kpad[0], Q.k[0], w.dwpart + P.w[0], grad + P.b[0], rows, w.ptotal, st);
+    return launch_tc_dw_accum(dcur, Q.n[0], w.x0, Q.kpad[0], Q.k[0], w.dwpart + P.w[0], grad + P.b[0], rows, w.ptotal, st);
   return launch_dw_accum(dcur, Q.n[0], w.x0, Q.kpad[0], Q.k[0], grad + P.w[0], grad + P.b[0], rows, st);
 }
 
@@ -562,8 +554,8 @@ int hb_value_grad(const hb_net_desc* d, const float* params, const float* prepar
 namespace {
 struct TrpoExtra { float* tprep; float* yd[2]; float* ttiles; };
 
-// tangent-prepared weights, two tangent activation buffers, GRU tangent buffers, and (experimental tensor-core tangent
-// block) the UMMA images of the tangent weights -- same size as the forward images
+// tangent-prepared weights, two tangent activation buffers, GRU tangent buffers, and (tensor-core tangent block) the
+// UMMA images of the tangent weights -- same size as the forward images
 size_t trpo_extra_floats(const hb::PrepLayout& Q, int64_t ch) {
   return (size_t)hb::round_up(Q.tk[0], 4) + 2 * (size_t)ch * hb::hmax_of(Q) + hb::rnn_jvp_floats(Q, ch) +
          (size_t)hb::round_up(Q.total - Q.tk[0], 4);
@@ -681,7 +673,7 @@ int hb_trpo_fvp(const hb_net_desc* d, const float* params, const float* prepared
     for (int l = 0; l < Lh; ++l) {
       float* yd = x.yd[l & 1];
       if (tc_jvp)
-        rc = launch_tc_jvp_linear_ln(gemm_impl() == 1 ? 3 : 1, d->activation, xin, ldx, xd, prepared + Q.tk[l],
+        rc = launch_tc_jvp_linear_ln(d->activation, xin, ldx, xd, prepared + Q.tk[l],
                                      x.ttiles + (Q.tk[l] - Q.tk[0]), Q.tk_chunks[l], x.tprep + Q.bias[l],
                                      prepared + Q.lnw[l], x.tprep + Q.lnw[l], x.tprep + Q.lnb[l], w.Z[l], w.stats[l], yd, n,
                                      Q.n[l], Q.kpad[l], st);
@@ -810,7 +802,7 @@ int hb_trpo_apply_step(float* params, const float* params0, const float* full_st
 }
 
 int hb_set_trpo_jvp_impl(int impl) {
-  HB_CHECK_ARG(impl == 0 || impl == 1, "impl must be 0 (FP32 FFMA tangent block) or 1 (experimental tcgen05 tangent block)");
+  HB_CHECK_ARG(impl == 0 || impl == 1, "impl must be 0 (FP32 FFMA tangent block) or 1 (tcgen05 tangent block)");
   g_trpo_jvp_impl.store(impl);
   return HB_OK;
 }
@@ -828,7 +820,7 @@ int hb_fused_timing_read(unsigned long long* out) {
 }
 
 int hb_set_rnn_impl(int impl) {
-  HB_CHECK_ARG(impl == 0 || impl == 1, "impl must be 0 (launch per step) or 1 (experimental persistent recurrence)");
+  HB_CHECK_ARG(impl == 0 || impl == 1, "impl must be 0 (launch per step) or 1 (persistent recurrence)");
   hb::set_rnn_impl(impl);
   return HB_OK;
 }

@@ -75,7 +75,7 @@ struct ParamLayout {
 };
 
 int make_layouts(const hb_net_desc* d, ParamLayout* pl, PrepLayout* pp, hb_net_layout* out);
-int gemm_impl();  // 0 = FP32 SIMT, 1 = tcgen05 3xTF32 (fp32-accurate), 2 = tcgen05 TF32
+int gemm_impl();  // 0 = FP32 SIMT, 1 = tcgen05 3xTF32 (fp32-accurate)
 
 // ------------------------------------------------------------------ device helpers
 #ifdef __CUDACC__
@@ -150,6 +150,29 @@ __device__ __forceinline__ float act_bwd_rt(int act, float z) {
     case HB_ACT_HARDSWISH: return act_bwd<HB_ACT_HARDSWISH>(z);
     default: return 1.f;
   }
+}
+
+// ValueNorm denormalisation of the returns kernels (valuenorm.py:38-45,78-92), every operation separately rounded as
+// in the reference: V^ = v * sqrt(max(E[v^2] - E[v]^2, 1e-2)) + E[v] with E[.] = running sum / max(debiasing term,
+// 1e-5).  vn == nullptr: no ValueNorm, V^ = v.
+struct VNConst { float mean, std; int on; };
+
+__device__ __forceinline__ VNConst vn_load(const float* __restrict__ vn) {
+  VNConst c;
+  c.on = vn != nullptr;
+  c.mean = 0.f;
+  c.std = 1.f;
+  if (c.on) {
+    float d = fmaxf(vn[2], 1e-5f);
+    float m = __fdiv_rn(vn[0], d), msq = __fdiv_rn(vn[1], d);
+    float var = fmaxf(__fsub_rn(msq, __fmul_rn(m, m)), 1e-2f);
+    c.mean = m;
+    c.std = __fsqrt_rn(var);
+  }
+  return c;
+}
+__device__ __forceinline__ float denorm(const VNConst& c, float v) {
+  return c.on ? __fadd_rn(__fmul_rn(v, c.std), c.mean) : v;
 }
 
 // gradient-sum output: a fire-and-forget reduction into this CTA's split-buffer slot (slot != 0: a handful of CTAs

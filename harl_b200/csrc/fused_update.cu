@@ -388,12 +388,9 @@ __global__ void __launch_bounds__(THREADS, 1) fused_update_kernel(const __grid_c
     um::mbar_init(m2e, 1);
     um::mbar_init(obs_free, 1);
     um::mbar_init(obs_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    um::fence_mbarrier_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(um::smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 0) um::tmem_alloc(tmem_slot, TMEM_COLS);
   um::fence_async_smem();
   um::tc_fence_before();
   __syncthreads();
@@ -925,7 +922,7 @@ __global__ void __launch_bounds__(THREADS, 1) fused_update_kernel(const __grid_c
   }
   um::tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS) : "memory");
+  if (warp == 0) um::tmem_dealloc(tmem, TMEM_COLS);
 }
 
 
@@ -990,12 +987,9 @@ __global__ void __launch_bounds__(THREADS, 1) fused_act_kernel(const __grid_cons
     um::mbar_init(e2m, 8);
     um::mbar_init(m2e, 1);
     um::mbar_init(obs_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    um::fence_mbarrier_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(um::smem_u32(tmem_slot)), "r"(ACT_TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 0) um::tmem_alloc(tmem_slot, ACT_TMEM_COLS);
   um::fence_async_smem();
   um::tc_fence_before();
   __syncthreads();
@@ -1166,7 +1160,7 @@ __global__ void __launch_bounds__(THREADS, 1) fused_act_kernel(const __grid_cons
   }
   um::tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(ACT_TMEM_COLS) : "memory");
+  if (warp == 0) um::tmem_dealloc(tmem, ACT_TMEM_COLS);
 }
 
 // ------------------------------------------------------------------------------------------------ weight images

@@ -10,41 +10,14 @@
 // four input arrays into shared memory with 16-byte cp.async (all loads in flight at once),
 // all threads form V^ = denorm(v) and delta_t in parallel, CW threads run the serial
 // recurrence out of shared memory, then all threads write returns/advantages coalesced.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace hb {
-
-// gae_tma.cu
-bool launch_gae_tma(const float* rewards, float* value_preds, const float* masks, const float* bad_masks,
-                    const float* next_value, float* returns, float* advantages, int T, int64_t C, float gamma, float gl,
-                    int ptl, const float* vn, cudaStream_t st, int* rc);
 
 // gae_seg.cu
 bool launch_gae_seg(const float* rewards, float* value_preds, const float* masks, const float* bad_masks,
                     const float* next_value, float* returns, float* advantages, int T, int64_t C, float gamma, float gl,
                     int ptl, const float* vn, cudaStream_t st, int* rc);
-
-struct VNConst { float mean, std; int on; };
-
-__device__ __forceinline__ VNConst vn_load(const float* __restrict__ vn) {
-  VNConst c;
-  c.on = vn != nullptr;
-  c.mean = 0.f;
-  c.std = 1.f;
-  if (c.on) {  // valuenorm.py:38-45,78-92
-    float d = fmaxf(vn[2], 1e-5f);
-    float m = __fdiv_rn(vn[0], d), msq = __fdiv_rn(vn[1], d);
-    float var = fmaxf(__fsub_rn(msq, __fmul_rn(m, m)), 1e-2f);
-    c.mean = m;
-    c.std = __fsqrt_rn(var);
-  }
-  return c;
-}
-__device__ __forceinline__ float denorm(const VNConst& c, float v) {
-  return c.on ? __fadd_rn(__fmul_rn(v, c.std), c.mean) : v;
-}
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
   unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
@@ -294,7 +267,7 @@ int hb_gae_returns(const float* rewards, float* value_preds, const float* masks,
   HB_CHECK_ARG(rewards && value_preds && masks && bad_masks && next_value && returns, "NULL buffer");
   HB_CHECK_ARG(T > 0 && C > 0, "T and C must be positive");
   cudaStream_t st = (cudaStream_t)stream;
-  if (use_gae) {  // register-resident, time-segmented kernel (gae_seg.cu): T <= 256 unless hb_set_gae_impl(0)
+  if (use_gae) {  // register-resident, time-segmented kernel (gae_seg.cu) for T <= 256
     int rc = HB_OK;
     if (hb::launch_gae_seg(rewards, value_preds, masks, bad_masks, next_value, returns, advantages, T, C, gamma, gamma_lambda,
                            use_proper_time_limits, vn_state, st, &rc))
@@ -309,14 +282,6 @@ int hb_gae_returns(const float* rewards, float* value_preds, const float* masks,
     for (int w : {32, 16, 8, 4}) {
       if (per_col * w <= budget && (cw == 0 || ceil_div64(C, cw) < 148)) cw = w;
     }
-    static const int forced = getenv("HB_GAE_CW") ? atoi(getenv("HB_GAE_CW")) : 0;   // tuning knob (4 / 8 / 16 / 32)
-    if ((forced == 4 || forced == 8 || forced == 16 || forced == 32) && per_col * forced <= budget) cw = forced;
-  }
-  if (use_gae && cw != 0) {  // TMA-staged kernel (gae_tma.cu); falls through to the cp.async kernel if it declines
-    int rc = HB_OK;
-    if (hb::launch_gae_tma(rewards, value_preds, masks, bad_masks, next_value, returns, advantages, T, C, gamma, gamma_lambda,
-                       use_proper_time_limits, vn_state, st, &rc))
-      return rc;
   }
 #define HB_GAE_TILED(W)                                                                                            \
   case W: {                                                                                                        \

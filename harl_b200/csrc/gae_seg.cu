@@ -1,4 +1,5 @@
-// GAE scan, time-segmented and register-resident (sm_100a): the default GAE branch of hb_gae_returns for T <= 256.
+// GAE scan, time-segmented and register-resident (sm_100a): the GAE branch of hb_gae_returns for T <= 256 (longer
+// rollouts run the tiled kernel of gae.cu).
 //
 // Same arithmetic as gae_tiled_kernel (gae.cu), i.e. OnPolicyCriticBuffer{EP,FP}.compute_returns
 // (harl/common/buffers/on_policy_critic_buffer_ep.py:97-140) + the advantage subtraction of
@@ -24,23 +25,6 @@
 #include "common.cuh"
 
 namespace hb {
-
-struct VNConstS { float mean, std; int on; };
-__device__ __forceinline__ VNConstS vn_load_s(const float* __restrict__ vn) {
-  VNConstS c;
-  c.on = vn != nullptr;
-  c.mean = 0.f;
-  c.std = 1.f;
-  if (c.on) {  // valuenorm.py:38-45,78-92
-    float d = fmaxf(vn[2], 1e-5f);
-    float m = __fdiv_rn(vn[0], d), msq = __fdiv_rn(vn[1], d);
-    float var = fmaxf(__fsub_rn(msq, __fmul_rn(m, m)), 1e-2f);
-    c.mean = m;
-    c.std = __fsqrt_rn(var);
-  }
-  return c;
-}
-__device__ __forceinline__ float denorm_s(const VNConstS& c, float v) { return c.on ? __fadd_rn(__fmul_rn(v, c.std), c.mean) : v; }
 
 __device__ __forceinline__ void named_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 __device__ __forceinline__ void named_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
@@ -84,10 +68,10 @@ __global__ void __launch_bounds__(32 * SEGS) gae_seg_kernel(const float* __restr
       if (PTL) bb[i] = 1.f;
     }
   }
-  const VNConstS vc = vn_load_s(vn);
-  vlast = denorm_s(vc, vlast);
+  const VNConst vc = vn_load(vn);
+  vlast = denorm(vc, vlast);
 #pragma unroll
-  for (int i = 0; i < L; ++i) vh[i] = denorm_s(vc, vh[i]);
+  for (int i = 0; i < L; ++i) vh[i] = denorm(vc, vh[i]);
 #pragma unroll
   for (int i = 0; i < L; ++i) {
     // delta = r + gamma * V^[t+1] * m[t+1] - V^[t];   am = gamma*lambda * m[t+1]
@@ -143,16 +127,15 @@ __global__ void __launch_bounds__(32 * SEGS) gae_seg_kernel(const float* __restr
   }
 }
 
-static int g_gae_impl = -1;   // 0 tiled (gae.cu), 1 segmented exact, 2 segmented scan
+// 1 = sequential carry (bit-exact), 2 = parallel-scan carry; -1: read HB_GAE_IMPL once (2, anything else gives 1)
+static int g_gae_impl = -1;
 int gae_impl() {
   if (g_gae_impl < 0) {
     const char* e = getenv("HB_GAE_IMPL");
-    g_gae_impl = e ? atoi(e) : 1;
-    if (g_gae_impl < 0 || g_gae_impl > 2) g_gae_impl = 1;
+    g_gae_impl = e != nullptr && atoi(e) == 2 ? 2 : 1;
   }
   return g_gae_impl;
 }
-void set_gae_impl(int v) { g_gae_impl = v < 0 || v > 2 ? 1 : v; }
 
 template <int SEGS, int L>
 static void launch_seg(bool ptl, bool scan, unsigned grid, cudaStream_t st, const float* rewards, float* value_preds,
@@ -165,23 +148,20 @@ static void launch_seg(bool ptl, bool scan, unsigned grid, cudaStream_t st, cons
 #undef HB_SEG
 }
 
-// Returns false if the shape is outside the kernel's range (the caller falls back to the tiled kernel).
+// Returns false if the shape is outside the kernel's range, T > 256 (the caller falls back to the tiled kernel).
 bool launch_gae_seg(const float* rewards, float* value_preds, const float* masks, const float* bad_masks, const float* next_value,
                     float* returns, float* advantages, int T, int64_t C, float gamma, float gl, int ptl, const float* vn,
                     cudaStream_t st, int* rc) {
-  const int impl = gae_impl();
-  if (impl == 0 || T > 256) return false;
-  const bool scan = impl == 2;
+  if (T > 256) return false;
+  const bool scan = gae_impl() == 2;
   const unsigned grid = (unsigned)ceil_div64(C, 32);
-  static const int forced = getenv("HB_GAE_SEGS") ? atoi(getenv("HB_GAE_SEGS")) : 0;   // tuning knob: 4 / 8 / 13
   // measured on B200 (profiles/gae_variants_r02.txt), T = 200: 13 segments x 16 steps wins for the sequential carry at
   // every width and for the scan below ~16k columns (shorter per-thread chains, 416 threads per CTA); 8 x 25 wins for
   // the scan on wide buffers (61 vs 84 us at 65536 columns: fewer, fatter threads keep more loads in flight per SM)
-  const bool seg13 = forced == 13 || (forced == 0 && T > 8 * 16 && T <= 13 * 16 && (!scan || C < 16384));
+  const bool seg13 = T > 8 * 16 && T <= 13 * 16 && (!scan || C < 16384);
 #define HB_GO(S, LL) launch_seg<S, LL>(ptl != 0, scan, grid, st, rewards, value_preds, masks, bad_masks, next_value, returns, \
                                        advantages, T, C, gamma, gl, vn)
-  if (seg13 && T <= 13 * 16) HB_GO(13, 16);
-  else if (forced == 4 && T <= 4 * 32) HB_GO(4, 32);
+  if (seg13) HB_GO(13, 16);
   else if (T <= 8 * 4) HB_GO(8, 4);
   else if (T <= 8 * 8) HB_GO(8, 8);
   else if (T <= 8 * 16) HB_GO(8, 16);
@@ -198,7 +178,8 @@ bool launch_gae_seg(const float* rewards, float* value_preds, const float* masks
 
 extern "C" {
 int hb_set_gae_impl(int impl) {
-  hb::set_gae_impl(impl);
+  HB_CHECK_ARG(impl == 1 || impl == 2, "impl must be 1 (sequential carry) or 2 (parallel scan)");
+  hb::g_gae_impl = impl;
   return HB_OK;
 }
 int hb_get_gae_impl(void) { return hb::gae_impl(); }

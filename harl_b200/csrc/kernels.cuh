@@ -75,17 +75,16 @@ int launch_ln_act_bwd(const float* dY, const float* Z, const float* stats, const
                       float* g_lnb, int64_t rows, int N, int act, cudaStream_t st);
 int launch_featnorm_fold(const hb_net_desc* d, const float* params, float* grad, cudaStream_t st);
 
-int launch_tc_linear_ln_fwd(int passes, int act, const float* X, int ldx, const float* tiles, int nchunks,
-                            const float* bias, const float* lnw, const float* lnb, float* Z, float* Y, float* stats,
+// tcgen05 3xTF32 layer-wise kernels (tc_gemm.cu)
+int launch_tc_linear_ln_fwd(int act, const float* X, int ldx, const float* tiles, int nchunks, const float* bias, const float* lnw, const float* lnb, float* Z, float* Y, float* stats,
                             int64_t M, int N, int Kred, cudaStream_t st);
-
-int launch_tc_dx_ln_bwd(int passes, int act, const float* dZ, int N, const float* tiles, int nchunks, const float* Zp,
+int launch_tc_dx_ln_bwd(int act, const float* dZ, int N, const float* tiles, int nchunks, const float* Zp,
                         const float* stats_p, const float* lnw_p, float* dZp, float* g_lnw_p, float* g_lnb_p, int64_t M,
                         int Np, int64_t part_delta, int64_t part_stride, cudaStream_t st);
-int launch_tc_dw_accum(int passes, const float* dZ, int N, const float* X, int ldx, int K, float* dW, float* db,
+int launch_tc_dw_accum(const float* dZ, int N, const float* X, int ldx, int K, float* dW, float* db,
                        int64_t M, int64_t part_stride, cudaStream_t st);
-// EXPERIMENTAL tensor-core tangent block (tc_gemm.cu), selected by hb_set_trpo_jvp_impl(1)
-int launch_tc_jvp_linear_ln(int passes, int act, const float* X, int ldx, const float* Xd, const float* tiles,
+// tensor-core tangent block, selected by hb_set_trpo_jvp_impl(1) (the default)
+int launch_tc_jvp_linear_ln(int act, const float* X, int ldx, const float* Xd, const float* tiles,
                             const float* tiles_d, int nchunks, const float* bd, const float* lnw, const float* lnwd,
                             const float* lnbd, const float* Z, const float* stats, float* Yd, int64_t M, int N, int Kred,
                             cudaStream_t st);

@@ -41,8 +41,6 @@ static int add_tensor(hb_net_layout* L, int* cursor, const char* name, int rows,
 // DiagGaussian (distributions.py:80-82): fc_mean registered before log_std is assigned, but
 // nn.Module yields own parameters (log_std) before sub-modules (fc_mean);  VNet: v_out.
 int tc_nt_of(int n);
-int launch_pack_umma_tiles(const float* W, int ldn, int ldk, const float* scale, int N, int K, int NT, int nchunks,
-                           float* dst, cudaStream_t st);
 int launch_pack_umma_jobs(int njobs, const float* const* W, const int* ldn, const int* ldk, const float* const* scale, const int* N,
                           const int* K, const int* NT, const int* nchunks, float* const* dst, cudaStream_t st);
 
@@ -193,7 +191,7 @@ __global__ void prepare_kernel(ParamLayout P, PrepLayout Q, int feature_norm, in
     if (i >= Q.lnw[l] && i < Q.lnw[l] + n) { prep[i] = params[P.lnw[l] + i - Q.lnw[l]]; return; }
     if (i >= Q.lnb[l] && i < Q.lnb[l] + n) { prep[i] = params[P.lnb[l] + i - Q.lnb[l]]; return; }
   }
-  if (i >= Q.tk[0]) return;  // tensor-core operand images are written by pack_umma_tiles
+  if (i >= Q.tk[0]) return;  // tensor-core operand images are written by pack_umma_jobs
   int h = Q.n[Q.n_layers - 1];
   if (i >= Q.hw && i < Q.hw + out_dim * h) { prep[i] = params[P.hw + i - Q.hw]; return; }
   if (i >= Q.hbias && i < Q.hbias + out_dim) { prep[i] = params[P.hbias + i - Q.hbias]; return; }
@@ -259,7 +257,7 @@ int hb_sync_check(void) {
 }
 
 int hb_set_gemm_impl(int impl) {
-  HB_CHECK_ARG(impl >= 0 && impl <= 2, "impl must be 0 (fp32 simt), 1 (tcgen05 3xtf32) or 2 (tcgen05 tf32)");
+  HB_CHECK_ARG(impl == 0 || impl == 1, "impl must be 0 (fp32 simt) or 1 (tcgen05 3xtf32)");
   hb::g_gemm_impl.store(impl);
   return HB_OK;
 }

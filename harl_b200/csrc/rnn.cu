@@ -166,14 +166,13 @@ __global__ void __launch_bounds__(ROW_THREADS) rnn_ln_fwd_kernel(const float* __
   }
 }
 
-// ------------------------------------------------------------------ persistent per-sequence recurrence (opt-in)
-// EXPERIMENTAL -- compiled, not yet run on a GPU (written after this round's GPU budget was spent); selected only by
-// hb_set_rnn_impl(1) / HB_RNN_IMPL=persistent, h = 64.  One warp owns one sequence for all S steps: W_hh^T (64 x 192
+// ------------------------------------------------------------------ persistent per-sequence recurrence (default)
+// hb_set_rnn_impl(1), the default, for h = 64 (other widths run the per-step kernels).  One warp owns one sequence for all S steps: W_hh^T (64 x 192
 // floats, regrouped so that lane l finds the r, z, n weights of its two hidden units 2l, 2l+1 in two LDS.128 per input
 // unit) stays in shared memory, the state stays in registers (unit i lives in lane i/2, broadcast by shuffle), and per
 // step the warp reads its gi row and the reset mask and writes hm / hs / gates exactly as the per-step kernels do.
 // Accumulation order matches the tiled GEMM (ascending input unit from zero, bias added last), so the results are
-// meant to be bit-identical to the launch-per-step path.  Replaces 2 S launches per layer by one.
+// bit-identical to the launch-per-step path (tests/test_gpu_rnn.py).  Replaces 2 S launches per layer by one.
 constexpr int GP_H = 64;
 __global__ void __launch_bounds__(256) gru_seq_fwd_kernel(const float* __restrict__ whh_t /* [64][192] */,
                                                           const float* __restrict__ bhh /* [192] */,
@@ -306,7 +305,7 @@ int rnn_forward(const PrepLayout& Q, const float* prep, const float* X, int64_t 
     if ((rc = launch_linear_plain(xin, h, prep + Q.rnn_wih_t[l], 3 * h, prep + Q.rnn_bih[l], w.gi[l], 3 * h, M, 3 * h, h,
                                   false, st)))
       return rc;
-    if (rnn_impl() == 1 && h == GP_H) {  // experimental persistent recurrence (see gru_seq_fwd_kernel)
+    if (rnn_impl() == 1 && h == GP_H) {  // persistent recurrence (see gru_seq_fwd_kernel)
       const size_t smem = (size_t)GP_H * 32 * 8 * sizeof(float);
       static bool attr_done = false;
       if (!attr_done) {

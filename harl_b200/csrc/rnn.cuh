@@ -29,7 +29,7 @@ struct RnnJvpWork {   // tangent pass of the trust-region Fisher-vector product
   float* outd;      // [M, h] tangent of LayerNorm(hs[top])
 };
 
-int rnn_impl();            // 0 = launch per step (default), 1 = experimental persistent per-sequence recurrence
+int rnn_impl();            // 0 = launch per step, 1 = persistent per-sequence recurrence (default; h = 64 only)
 void set_rnn_impl(int v);
 size_t rnn_jvp_floats(const PrepLayout& Q, int64_t M);
 int carve_rnn_jvp(const PrepLayout& Q, int64_t M, float* p, RnnJvpWork* w);

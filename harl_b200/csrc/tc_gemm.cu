@@ -2,10 +2,10 @@
 //
 //   tc_linear_ln_fwd : Y = LN(act(X W'^T + b'))     (same contract as the SIMT linear_ln_fwd_kernel)
 //
-// Numerics: kind::tf32 MMAs with fp32 accumulation in TMEM.  PASSES = 3 runs the error-compensated
-// split  x = hi + lo  (hi = x rounded to TF32, lo = the residual rounded to TF32, both exactly
-// representable in TF32 up to 2^-22):  D += A_hi B_hi + A_lo B_hi + A_hi B_lo, which restores fp32-level
-// accuracy (relative error ~3e-7 per product) at 3 MMAs per tile; PASSES = 1 is plain TF32.
+// Numerics: kind::tf32 MMAs with fp32 accumulation in TMEM, error-compensated: x = hi + lo (hi = x rounded to TF32,
+// lo = the residual rounded to TF32, both exactly representable in TF32 up to 2^-22) and
+// D += A_hi B_hi + A_lo B_hi + A_hi B_lo, which restores fp32-level accuracy (relative error ~3e-7 per product) at
+// 3 MMAs per k-step.
 //
 // Structure of one CTA (128 threads = 4 warps, one 128-row tile, UMMA 128 x NT x 8):
 //   * operands live in shared memory in the canonical K-major no-swizzle UMMA layout
@@ -19,6 +19,7 @@
 //     LayerNorm row statistics are thread-local: three passes over TMEM (sum, centred sum of squares, write).
 #include "common.cuh"
 #include "kernels.cuh"
+#include "umma.cuh"
 
 namespace hb {
 
@@ -28,70 +29,6 @@ constexpr int TC_KC = 32;    // floats of K per pipeline stage (4 MMA k-steps)
 // loads / epilogue overlap the others' MMAs -- inter-CTA instead of intra-CTA pipelining.
 constexpr int TC_STAGES = 1;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void tma_bulk_g2s(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// K-major, SWIZZLE_NONE shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout, version 1)
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = (uint64_t)((saddr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= (uint64_t)1 << 46;
-  return d;
-}
-// instruction descriptor: D fp32, A/B tf32, both K-major, M = 128, N = n
-__host__ __device__ constexpr uint32_t umma_idesc_tf32(int n) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
 // Round-to-nearest TF32 (cvt.rna): |x - hi| <= 2^-11 |x| and, for the residual, |r - lo| <= 2^-11 |r|, so
 // x = hi + lo up to 2^-22 |x| -- four times tighter than clearing the low 13 mantissa bits, at the same MMA count.
 // (two integer ops: add half a TF32 ulp to the magnitude bits, clear the low 13; a mantissa carry into the exponent
@@ -100,32 +37,8 @@ __device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float((__fl
 __device__ __forceinline__ float tf32_lo(float x, float hi) { return tf32_hi(x - hi); }
 
 // ------------------------------------------------------------------ weight tile packing (part of hb_net_prepare)
-// dst: for each k-chunk c (32 wide): hi image [NT][32] then lo image, canonical K-major UMMA layout.
+// Per job: for each k-chunk c (32 wide), hi image [NT][32] then lo image, canonical K-major UMMA layout;
 // src(n, k) = W[n*ldn + k*ldk] * (scale ? scale[k] : 1), zero outside [N) x [K).
-__global__ void pack_umma_tiles_kernel(const float* __restrict__ W, int ldn, int ldk, const float* __restrict__ scale,
-                                       int N, int K, int NT, int nchunks, float* __restrict__ dst) {
-  const int per_chunk = 2 * NT * TC_KC;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nchunks * NT * TC_KC; i += gridDim.x * blockDim.x) {
-    const int c = i / (NT * TC_KC), e = i % (NT * TC_KC);
-    // e indexes the image: [(n/8)][kc (8)][n%8][4]
-    const int k4 = e & 3, n8 = (e >> 2) & 7, kc = (e >> 5) & 7, ng = e >> 8;
-    const int n = ng * 8 + n8, k = c * TC_KC + kc * 4 + k4;
-    float v = 0.f;
-    if (n < N && k < K) { v = W[(int64_t)n * ldn + (int64_t)k * ldk]; if (scale) v *= scale[k]; }
-    const float hi = tf32_hi(v);
-    dst[(int64_t)c * per_chunk + e] = hi;
-    dst[(int64_t)c * per_chunk + NT * TC_KC + e] = tf32_lo(v, hi);
-  }
-}
-
-int launch_pack_umma_tiles(const float* W, int ldn, int ldk, const float* scale, int N, int K, int NT, int nchunks,
-                           float* dst, cudaStream_t st) {
-  int total = nchunks * NT * TC_KC;
-  pack_umma_tiles_kernel<<<(total + 255) / 256, 256, 0, st>>>(W, ldn, ldk, scale, N, K, NT, nchunks, dst);
-  HB_LAUNCH_DONE(st, "pack_umma_tiles");
-  return HB_OK;
-}
-
 // All images of one net in ONE launch (blockIdx.y = job): hb_net_prepare runs after every optimiser step, and three
 // 3-6 us launches per net were 2 % of the C2 update phase.
 struct PackUmmaJobs {
@@ -144,6 +57,7 @@ __global__ void pack_umma_jobs_kernel(const __grid_constant__ PackUmmaJobs J) {
   const int per_chunk = 2 * NT * TC_KC;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < J.nchunks[j] * NT * TC_KC; i += gridDim.x * blockDim.x) {
     const int c = i / (NT * TC_KC), e = i % (NT * TC_KC);
+    // e indexes the image: [(n/8)][kc (8)][n%8][4]
     const int k4 = e & 3, n8 = (e >> 2) & 7, kc = (e >> 5) & 7, ng = e >> 8;
     const int n = ng * 8 + n8, k = c * TC_KC + kc * 4 + k4;
     float v = 0.f;
@@ -171,6 +85,11 @@ int launch_pack_umma_jobs(int njobs, const float* const* W, const int* ldn, cons
   return HB_OK;
 }
 
+int launch_pack_umma_tiles(const float* W, int ldn, int ldk, const float* scale, int N, int K, int NT, int nchunks,
+                           float* dst, cudaStream_t st) {
+  return launch_pack_umma_jobs(1, &W, &ldn, &ldk, &scale, &N, &K, &NT, &nchunks, &dst, st);
+}
+
 // ------------------------------------------------------------------ forward block on tcgen05
 template <int NT>
 struct TcSmem {
@@ -185,7 +104,84 @@ struct TcSmem {
   alignas(16) float plnb[NT];
 };
 
-template <int NT, int ACT, int PASSES>
+// One operand chunk of the mainloop: A = this thread's tile row from its first column of the chunk on (`k` of its 32
+// columns are valid, the rest are staged as zeros), B = the chunk's pre-packed hi + lo weight image.
+struct TcChunk {
+  const float* a;
+  int k;
+  const float* b;
+};
+
+// Setup and mainloop shared by the forward, dX and tangent kernels: allocates NT TMEM columns and accumulates
+// acc[128 x NT] = sum over n chunks of A_c B_c^T (3xTF32), with chunk(c) naming the operands of chunk c.  Returns the
+// TMEM base address once every MMA has retired; the caller frees it with um::tmem_dealloc.
+template <int NT, class ChunkOf>
+__device__ __forceinline__ uint32_t tc_mainloop(TcSmem<NT>& s, int tid, bool row_ok, int n, ChunkOf&& chunk) {
+  constexpr uint32_t B_BYTES = 2u * NT * TC_KC * sizeof(float);
+  if (tid == 0) {
+    for (int i = 0; i < TC_STAGES; ++i) { um::mbar_init(&s.full_b[i], 1); um::mbar_init(&s.empty[i], 1); }
+    um::mbar_init(&s.done, 1);
+    um::fence_mbarrier_init();
+  }
+  if ((tid >> 5) == 0) um::tmem_alloc(&s.tmem_base, NT);
+  um::tc_fence_before();
+  __syncthreads();
+  um::tc_fence_after();
+  const uint32_t tmem = s.tmem_base;
+  constexpr uint32_t idesc = um::idesc_tf32(NT);
+
+  uint32_t ph_full[2] = {0, 0}, ph_empty[2] = {0, 0};
+  for (int c = 0; c < n; ++c) {
+    const int st = c % TC_STAGES;
+    if (c >= TC_STAGES) { um::mbar_wait(&s.empty[st], ph_empty[st]); ph_empty[st] ^= 1; }  // stage free again
+    // chunk(c) is evaluated where each part is used: a B pointer formed outside the thread-0 branch costs every
+    // thread two registers
+    if (tid == 0) {
+      um::mbar_expect_tx(&s.full_b[st], B_BYTES);
+      um::tma_bulk_g2s(s.b[st], chunk(c).b, B_BYTES, &s.full_b[st]);
+    }
+    // A: thread t stages row t of the tile (zeros beyond M / the valid columns), hi and lo images
+    {
+      const TcChunk ch = chunk(c);
+      float* ahi = s.a[st][0];
+      float* alo = s.a[st][1];
+      const int base = ((tid >> 3) * 8) * 32 + (tid & 7) * 4;  // floats: [(row/8)][kc][row%8][4]
+#pragma unroll
+      for (int kc = 0; kc < 8; ++kc) {
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (row_ok && kc * 4 < ch.k) v = *reinterpret_cast<const float4*>(ch.a + kc * 4);
+        float4 h = make_float4(tf32_hi(v.x), tf32_hi(v.y), tf32_hi(v.z), tf32_hi(v.w));
+        *reinterpret_cast<float4*>(ahi + base + kc * 32) = h;
+        *reinterpret_cast<float4*>(alo + base + kc * 32) = make_float4(tf32_lo(v.x, h.x), tf32_lo(v.y, h.y), tf32_lo(v.z, h.z), tf32_lo(v.w, h.w));
+      }
+    }
+    um::fence_async_smem();   // generic-proxy smem writes -> visible to the tensor core (async proxy)
+    __syncthreads();
+    if (tid == 0) {
+      um::mbar_wait(&s.full_b[st], ph_full[st]);
+      um::tc_fence_after();
+      const uint32_t a_hi = um::smem_u32(s.a[st][0]), a_lo = um::smem_u32(s.a[st][1]);
+      const uint32_t b_hi = um::smem_u32(s.b[st]), b_lo = b_hi + NT * TC_KC * sizeof(float);
+#pragma unroll
+      for (int j = 0; j < TC_KC / 8; ++j) {
+        const uint32_t off = j * 256;
+        const uint64_t dah = um::desc(a_hi + off, 128, 1024), dbh = um::desc(b_hi + off, 128, 1024);
+        um::mma_tf32(tmem, dah, dbh, idesc, (c | j) != 0);
+        const uint64_t dal = um::desc(a_lo + off, 128, 1024), dbl = um::desc(b_lo + off, 128, 1024);
+        um::mma_tf32(tmem, dal, dbh, idesc, 1);
+        um::mma_tf32(tmem, dah, dbl, idesc, 1);
+      }
+      um::commit(&s.empty[st]);            // arrives when the MMAs above have finished reading this stage
+      if (c == n - 1) um::commit(&s.done);
+    }
+    ph_full[st] ^= 1;
+  }
+  um::mbar_wait(&s.done, 0);
+  um::tc_fence_after();
+  return tmem;
+}
+
+template <int NT, int ACT>
 __global__ void __launch_bounds__(128, 1) tc_linear_ln_fwd_kernel(const float* __restrict__ X, int ldx,
                                                                   const float* __restrict__ tiles, int nchunks,
                                                                   const float* __restrict__ bias,
@@ -198,76 +194,15 @@ __global__ void __launch_bounds__(128, 1) tc_linear_ln_fwd_kernel(const float* _
   const int tid = threadIdx.x, warp = tid >> 5;
   const int64_t row0 = (int64_t)blockIdx.x * TC_BM;
   const int64_t row = row0 + tid;
-  constexpr uint32_t B_BYTES = 2u * NT * TC_KC * sizeof(float);
 
   for (int i = tid; i < NT; i += 128) {
     s.pbias[i] = i < N ? bias[i] : 0.f;
     s.plnw[i] = i < N ? lnw[i] : 0.f;
     s.plnb[i] = i < N ? lnb[i] : 0.f;
   }
-  if (tid == 0) {
-    for (int i = 0; i < TC_STAGES; ++i) { mbar_init(&s.full_b[i], 1); mbar_init(&s.empty[i], 1); }
-    mbar_init(&s.done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s.tmem_base)), "r"((uint32_t)NT) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = s.tmem_base;
-  constexpr uint32_t idesc = umma_idesc_tf32(NT);
-
-  uint32_t ph_full[2] = {0, 0}, ph_empty[2] = {0, 0};
-  for (int c = 0; c < nchunks; ++c) {
-    const int st = c % TC_STAGES;
-    if (c >= TC_STAGES) { mbar_wait(&s.empty[st], ph_empty[st]); ph_empty[st] ^= 1; }  // stage free again
-    if (tid == 0) {
-      mbar_expect_tx(&s.full_b[st], B_BYTES);
-      tma_bulk_g2s(s.b[st], tiles + (int64_t)c * (2 * NT * TC_KC), B_BYTES, &s.full_b[st]);
-    }
-    // A: thread t stages row t of the tile (zeros beyond M / Kred), hi and lo images
-    {
-      float* ahi = s.a[st][0];
-      float* alo = s.a[st][1];
-      const int base = ((tid >> 3) * 8) * 32 + (tid & 7) * 4;  // floats: [(row/8)][kc][row%8][4]
-      const float* xr = X + row * ldx + c * TC_KC;
-#pragma unroll
-      for (int kc = 0; kc < 8; ++kc) {
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (row < M && c * TC_KC + kc * 4 < Kred) v = *reinterpret_cast<const float4*>(xr + kc * 4);
-        float4 h = make_float4(tf32_hi(v.x), tf32_hi(v.y), tf32_hi(v.z), tf32_hi(v.w));
-        *reinterpret_cast<float4*>(ahi + base + kc * 32) = h;
-        if (PASSES == 3) *reinterpret_cast<float4*>(alo + base + kc * 32) = make_float4(tf32_lo(v.x, h.x), tf32_lo(v.y, h.y), tf32_lo(v.z, h.z), tf32_lo(v.w, h.w));
-      }
-    }
-    fence_async_smem();   // generic-proxy smem writes -> visible to the tensor core (async proxy)
-    __syncthreads();
-    if (tid == 0) {
-      mbar_wait(&s.full_b[st], ph_full[st]);
-      tc_fence_after();
-      const uint32_t a_hi = smem_u32(s.a[st][0]), a_lo = smem_u32(s.a[st][1]);
-      const uint32_t b_hi = smem_u32(s.b[st]), b_lo = b_hi + NT * TC_KC * sizeof(float);
-#pragma unroll
-      for (int j = 0; j < TC_KC / 8; ++j) {
-        const uint32_t off = j * 256;
-        const uint64_t dah = umma_desc(a_hi + off, 128, 1024), dbh = umma_desc(b_hi + off, 128, 1024);
-        umma_tf32(tmem, dah, dbh, idesc, (c | j) != 0);
-        if (PASSES == 3) {
-          const uint64_t dal = umma_desc(a_lo + off, 128, 1024), dbl = umma_desc(b_lo + off, 128, 1024);
-          umma_tf32(tmem, dal, dbh, idesc, 1);
-          umma_tf32(tmem, dah, dbl, idesc, 1);
-        }
-      }
-      umma_commit(&s.empty[st]);            // arrives when the MMAs above have finished reading this stage
-      if (c == nchunks - 1) umma_commit(&s.done);
-    }
-    ph_full[st] ^= 1;
-  }
-  mbar_wait(&s.done, 0);
-  tc_fence_after();
+  const uint32_t tmem = tc_mainloop(s, tid, row < M, nchunks, [&](int c) {
+    return TcChunk{X + row * ldx + c * TC_KC, Kred - c * TC_KC, tiles + (int64_t)c * (2 * NT * TC_KC)};
+  });
 
   // ---- epilogue: thread = row.  z = acc + b, a = act(z), LayerNorm over the N valid columns.
   // Three passes over the accumulator row in TMEM: sum, centred sum of squares (the exact two-pass LayerNorm
@@ -281,7 +216,7 @@ __global__ void __launch_bounds__(128, 1) tc_linear_ln_fwd_kernel(const float* _
   float sum = 0.f;
   for (int c0 = 0; c0 < N; c0 += 32) {
     float v[32];
-    tmem_ld32(trow + c0, v);
+    um::tmem_ld32(trow + c0, v);
 #pragma unroll
     for (int j4 = 0; j4 < 32; j4 += 4) {
       if (c0 + j4 < N) {  // N is a multiple of 4
@@ -297,7 +232,7 @@ __global__ void __launch_bounds__(128, 1) tc_linear_ln_fwd_kernel(const float* _
   float sq = 0.f;
   for (int c0 = 0; c0 < N; c0 += 32) {
     float v[32];
-    tmem_ld32(trow + c0, v);
+    um::tmem_ld32(trow + c0, v);
 #pragma unroll
     for (int j4 = 0; j4 < 32; j4 += 4) {
       if (c0 + j4 < N) {
@@ -323,7 +258,7 @@ __global__ void __launch_bounds__(128, 1) tc_linear_ln_fwd_kernel(const float* _
   for (int h = 0; h < NH; ++h) {
     for (int c0 = h * HC; c0 < (h + 1) * HC && c0 < N; c0 += 32) {
       float v[32];
-      tmem_ld32(trow + c0, v);
+      um::tmem_ld32(trow + c0, v);
 #pragma unroll
       for (int j4 = 0; j4 < 32; j4 += 4) {
         if (c0 + j4 < N && c0 + j4 < (h + 1) * HC) {
@@ -360,12 +295,12 @@ __global__ void __launch_bounds__(128, 1) tc_linear_ln_fwd_kernel(const float* _
   }
   if (stats != nullptr && row < M) { stats[row * 2] = mean; stats[row * 2 + 1] = rstd; }
 
-  tc_fence_before();
+  um::tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)NT) : "memory");
+  if (warp == 0) um::tmem_dealloc(tmem, NT);
 }
 
-template <int NT, int PASSES>
+template <int NT>
 static int launch_tc_fwd_nt(int act, const float* X, int ldx, const float* tiles, int nchunks, const float* bias,
                             const float* lnw, const float* lnb, float* Z, float* Y, float* stats, int64_t M, int N,
                             int Kred, cudaStream_t st) {
@@ -373,7 +308,7 @@ static int launch_tc_fwd_nt(int act, const float* X, int ldx, const float* tiles
   dim3 grid((unsigned)ceil_div64(M, TC_BM));
 #define HB_TC_CASE(A)                                                                                       \
   case A: {                                                                                                 \
-    auto kern = tc_linear_ln_fwd_kernel<NT, A, PASSES>;                                                     \
+    auto kern = tc_linear_ln_fwd_kernel<NT, A>;                                                             \
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                     \
     kern<<<grid, 128, smem, st>>>(X, ldx, tiles, nchunks, bias, lnw, lnb, Z, Y, stats, M, N, Kred);         \
   } break;
@@ -383,21 +318,20 @@ static int launch_tc_fwd_nt(int act, const float* X, int ldx, const float* tiles
     default: set_error("activation %d", act); return HB_ERR_UNSUPPORTED;
   }
 #undef HB_TC_CASE
-  HB_LAUNCH_DONE(st, shape_label(PASSES == 3 ? "tc_linear_ln_fwd_3xtf32" : "tc_linear_ln_fwd_tf32", M, N, Kred));
+  HB_LAUNCH_DONE(st, shape_label("tc_linear_ln_fwd_3xtf32", M, N, Kred));
   return HB_OK;
 }
 
 int tc_nt_of(int n) { return n <= 32 ? 32 : n <= 64 ? 64 : n <= 128 ? 128 : 256; }
 
-int launch_tc_linear_ln_fwd(int passes, int act, const float* X, int ldx, const float* tiles, int nchunks,
+int launch_tc_linear_ln_fwd(int act, const float* X, int ldx, const float* tiles, int nchunks,
                             const float* bias, const float* lnw, const float* lnb, float* Z, float* Y, float* stats,
                             int64_t M, int N, int Kred, cudaStream_t st) {
   if (M <= 0) return HB_OK;
   const int nt = tc_nt_of(N);
 #define HB_TC_NT(NTV)                                                                                              \
   case NTV:                                                                                                        \
-    return passes == 3 ? launch_tc_fwd_nt<NTV, 3>(act, X, ldx, tiles, nchunks, bias, lnw, lnb, Z, Y, stats, M, N, Kred, st) \
-                       : launch_tc_fwd_nt<NTV, 1>(act, X, ldx, tiles, nchunks, bias, lnw, lnb, Z, Y, stats, M, N, Kred, st);
+    return launch_tc_fwd_nt<NTV>(act, X, ldx, tiles, nchunks, bias, lnw, lnb, Z, Y, stats, M, N, Kred, st);
   switch (nt) { HB_TC_NT(32) HB_TC_NT(64) HB_TC_NT(128) HB_TC_NT(256) }
 #undef HB_TC_NT
   return HB_ERR_UNSUPPORTED;
@@ -430,7 +364,7 @@ __device__ __forceinline__ float warp_colsum32(float (&v)[32], int lane) {
 }
 
 // ---- dYp = dZ [M,N] W [N,Np] on tensor cores, then LN-backward + act' of the previous block (thread = row)
-template <int NT, int ACT, int PASSES>
+template <int NT, int ACT>
 __global__ void __launch_bounds__(128, 1) tc_dx_ln_bwd_kernel(const float* __restrict__ dZ, int N,
                                                               const float* __restrict__ tiles, int nchunks,
                                                               const float* __restrict__ Zp, const float* __restrict__ stats_p,
@@ -442,68 +376,9 @@ __global__ void __launch_bounds__(128, 1) tc_dx_ln_bwd_kernel(const float* __res
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int64_t row0 = (int64_t)blockIdx.x * TC_BM;
   const int64_t row = row0 + tid;
-  constexpr uint32_t B_BYTES = 2u * NT * TC_KC * sizeof(float);
-  if (tid == 0) {
-    for (int i = 0; i < TC_STAGES; ++i) { mbar_init(&s.full_b[i], 1); mbar_init(&s.empty[i], 1); }
-    mbar_init(&s.done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s.tmem_base)), "r"((uint32_t)NT) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = s.tmem_base;
-  constexpr uint32_t idesc = umma_idesc_tf32(NT);
-  uint32_t ph_full[2] = {0, 0}, ph_empty[2] = {0, 0};
-  for (int c = 0; c < nchunks; ++c) {
-    const int st = c % TC_STAGES;
-    if (c >= TC_STAGES) { mbar_wait(&s.empty[st], ph_empty[st]); ph_empty[st] ^= 1; }
-    if (tid == 0) {
-      mbar_expect_tx(&s.full_b[st], B_BYTES);
-      tma_bulk_g2s(s.b[st], tiles + (int64_t)c * (2 * NT * TC_KC), B_BYTES, &s.full_b[st]);
-    }
-    {
-      float* ahi = s.a[st][0];
-      float* alo = s.a[st][1];
-      const int base = ((tid >> 3) * 8) * 32 + (tid & 7) * 4;
-      const float* xr = dZ + row * N + c * TC_KC;
-#pragma unroll
-      for (int kc = 0; kc < 8; ++kc) {
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (row < M && c * TC_KC + kc * 4 < N) v = *reinterpret_cast<const float4*>(xr + kc * 4);
-        float4 h = make_float4(tf32_hi(v.x), tf32_hi(v.y), tf32_hi(v.z), tf32_hi(v.w));
-        *reinterpret_cast<float4*>(ahi + base + kc * 32) = h;
-        if (PASSES == 3) *reinterpret_cast<float4*>(alo + base + kc * 32) = make_float4(tf32_lo(v.x, h.x), tf32_lo(v.y, h.y), tf32_lo(v.z, h.z), tf32_lo(v.w, h.w));
-      }
-    }
-    fence_async_smem();
-    __syncthreads();
-    if (tid == 0) {
-      mbar_wait(&s.full_b[st], ph_full[st]);
-      tc_fence_after();
-      const uint32_t a_hi = smem_u32(s.a[st][0]), a_lo = smem_u32(s.a[st][1]);
-      const uint32_t b_hi = smem_u32(s.b[st]), b_lo = b_hi + NT * TC_KC * sizeof(float);
-#pragma unroll
-      for (int j = 0; j < TC_KC / 8; ++j) {
-        const uint32_t off = j * 256;
-        const uint64_t dah = umma_desc(a_hi + off, 128, 1024), dbh = umma_desc(b_hi + off, 128, 1024);
-        umma_tf32(tmem, dah, dbh, idesc, (c | j) != 0);
-        if (PASSES == 3) {
-          const uint64_t dal = umma_desc(a_lo + off, 128, 1024), dbl = umma_desc(b_lo + off, 128, 1024);
-          umma_tf32(tmem, dal, dbh, idesc, 1);
-          umma_tf32(tmem, dah, dbl, idesc, 1);
-        }
-      }
-      umma_commit(&s.empty[st]);
-      if (c == nchunks - 1) umma_commit(&s.done);
-    }
-    ph_full[st] ^= 1;
-  }
-  mbar_wait(&s.done, 0);
-  tc_fence_after();
+  const uint32_t tmem = tc_mainloop(s, tid, row < M, nchunks, [&](int c) {
+    return TcChunk{dZ + row * N + c * TC_KC, N - c * TC_KC, tiles + (int64_t)c * (2 * NT * TC_KC)};
+  });
 
   // ---- epilogue.  Parameters / column sums live in the small shared arrays; the Zp tile is staged through the (now
   // idle) operand stage with coalesced loads and an XOR chunk swizzle, transformed in place into dZp by its row's
@@ -532,7 +407,7 @@ __global__ void __launch_bounds__(128, 1) tc_dx_ln_bwd_kernel(const float* __res
   float s1 = 0.f, s2 = 0.f;
   for (int c0 = 0; c0 < Np; c0 += 32) {
     float v[32], cg[32], cb[32];
-    tmem_ld32(trow + c0, v);
+    um::tmem_ld32(trow + c0, v);
 #pragma unroll
     for (int j4 = 0; j4 < 32; j4 += 4) {
       float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -559,7 +434,7 @@ __global__ void __launch_bounds__(128, 1) tc_dx_ln_bwd_kernel(const float* __res
   const float m1 = s1 * inv_n, m2 = s2 * inv_n;
   for (int c0 = 0; c0 < Np; c0 += 32) {
     float v[32];
-    tmem_ld32(trow + c0, v);
+    um::tmem_ld32(trow + c0, v);
 #pragma unroll
     for (int j4 = 0; j4 < 32; j4 += 4) {
       if (c0 + j4 < Np) {
@@ -596,12 +471,12 @@ __global__ void __launch_bounds__(128, 1) tc_dx_ln_bwd_kernel(const float* __res
     const int64_t slot = part_stride ? part_delta + (int64_t)(blockIdx.x % (unsigned)tc_dw_splits_c()) * part_stride : 0;
     for (int n = tid; n < Np; n += 128) { acc_out(g_lnw_p + n, colsum[n], slot); acc_out(g_lnb_p + n, colsum[NT + n], slot); }
   }
-  tc_fence_before();
+  um::tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)NT) : "memory");
+  if (warp == 0) um::tmem_dealloc(tmem, NT);
 }
 
-template <int NT, int PASSES>
+template <int NT>
 static int launch_tc_dx_nt(int act, const float* dZ, int N, const float* tiles, int nchunks, const float* Zp,
                            const float* stats_p, const float* lnw_p, float* dZp, float* g_lnw_p, float* g_lnb_p,
                            int64_t M, int Np, int64_t part_delta, int64_t part_stride, cudaStream_t st) {
@@ -609,7 +484,7 @@ static int launch_tc_dx_nt(int act, const float* dZ, int N, const float* tiles, 
   dim3 grid((unsigned)ceil_div64(M, TC_BM));
 #define HB_TC_CASE(A)                                                                                       \
   case A: {                                                                                                 \
-    auto kern = tc_dx_ln_bwd_kernel<NT, A, PASSES>;                                                         \
+    auto kern = tc_dx_ln_bwd_kernel<NT, A>;                                                                 \
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                     \
     kern<<<grid, 128, smem, st>>>(dZ, N, tiles, nchunks, Zp, stats_p, lnw_p, dZp, g_lnw_p, g_lnb_p, M, Np, part_delta, part_stride); \
   } break;
@@ -619,32 +494,31 @@ static int launch_tc_dx_nt(int act, const float* dZ, int N, const float* tiles, 
     default: set_error("activation %d", act); return HB_ERR_UNSUPPORTED;
   }
 #undef HB_TC_CASE
-  HB_LAUNCH_DONE(st, shape_label(PASSES == 3 ? "tc_dx_ln_bwd_3xtf32" : "tc_dx_ln_bwd_tf32", M, Np, N));
+  HB_LAUNCH_DONE(st, shape_label("tc_dx_ln_bwd_3xtf32", M, Np, N));
   return HB_OK;
 }
 
-int launch_tc_dx_ln_bwd(int passes, int act, const float* dZ, int N, const float* tiles, int nchunks, const float* Zp,
+int launch_tc_dx_ln_bwd(int act, const float* dZ, int N, const float* tiles, int nchunks, const float* Zp,
                         const float* stats_p, const float* lnw_p, float* dZp, float* g_lnw_p, float* g_lnb_p, int64_t M,
                         int Np, int64_t part_delta, int64_t part_stride, cudaStream_t st) {
   if (M <= 0) return HB_OK;
 #define HB_TC_NT(NTV)                                                                                                   \
   case NTV:                                                                                                             \
-    return passes == 3 ? launch_tc_dx_nt<NTV, 3>(act, dZ, N, tiles, nchunks, Zp, stats_p, lnw_p, dZp, g_lnw_p, g_lnb_p, M, Np, part_delta, part_stride, st) \
-                       : launch_tc_dx_nt<NTV, 1>(act, dZ, N, tiles, nchunks, Zp, stats_p, lnw_p, dZp, g_lnw_p, g_lnb_p, M, Np, part_delta, part_stride, st);
+    return launch_tc_dx_nt<NTV>(act, dZ, N, tiles, nchunks, Zp, stats_p, lnw_p, dZp, g_lnw_p, g_lnb_p, M, Np, part_delta, part_stride, st);
   switch (tc_nt_of(Np)) { HB_TC_NT(32) HB_TC_NT(64) HB_TC_NT(128) HB_TC_NT(256) }
 #undef HB_TC_NT
   return HB_ERR_UNSUPPORTED;
 }
 
-// ---- EXPERIMENTAL (compiled, not yet run on a GPU; opt-in through hb_set_trpo_jvp_impl(1)): tangent of one
-// Linear -> act -> LayerNorm block on tensor cores, for the trust-region Fisher-vector product (trpo.cu).
+// ---- Tangent of one Linear -> act -> LayerNorm block on tensor cores, for the trust-region Fisher-vector product
+// (trpo.cu; the default tangent block, hb_set_trpo_jvp_impl(1)).
 //   acc = Xd W^T + X Wd^T  as ONE accumulation over 2 x nchunks operand chunks (phase 0: A = Xd, B = the forward
 //   weight images; phase 1: A = X, B = images of the tangent weights packed per product by pack_umma_tiles), then
 //   ad = act'(Z) (acc + bd);  xh = (act(Z) - mu) rstd;  yd = gd xh + betad + g rstd (ad - mean(ad) - xh mean(xh ad)).
-// Mainloop and Z-tile staging are those of tc_dx_ln_bwd_kernel (thread = row in the epilogue); pbias <- bd, plnw <- g,
+// Z-tile staging is that of tc_dx_ln_bwd_kernel (thread = row in the epilogue); pbias <- bd, plnw <- g,
 // plnb <- gd, betad is read from global memory (broadcast).  Xd == nullptr (first layer: the normalised observations
 // carry no tangent) runs phase 1 only.
-template <int NT, int ACT, int PASSES>
+template <int NT, int ACT>
 __global__ void __launch_bounds__(128, 1) tc_jvp_linear_ln_kernel(const float* __restrict__ X, int ldx,
                                                                   const float* __restrict__ Xd,
                                                                   const float* __restrict__ tiles,
@@ -658,77 +532,19 @@ __global__ void __launch_bounds__(128, 1) tc_jvp_linear_ln_kernel(const float* _
   const int tid = threadIdx.x, warp = tid >> 5;
   const int64_t row0 = (int64_t)blockIdx.x * TC_BM;
   const int64_t row = row0 + tid;
-  constexpr uint32_t B_BYTES = 2u * NT * TC_KC * sizeof(float);
   for (int i = tid; i < NT; i += 128) {
     s.pbias[i] = i < Np ? bd[i] : 0.f;
     s.plnw[i] = i < Np ? lnw[i] : 0.f;
     s.plnb[i] = i < Np ? lnwd[i] : 0.f;
   }
-  if (tid == 0) {
-    for (int i = 0; i < TC_STAGES; ++i) { mbar_init(&s.full_b[i], 1); mbar_init(&s.empty[i], 1); }
-    mbar_init(&s.done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s.tmem_base)), "r"((uint32_t)NT) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = s.tmem_base;
-  constexpr uint32_t idesc = umma_idesc_tf32(NT);
-  uint32_t ph_full[2] = {0, 0}, ph_empty[2] = {0, 0};
   const int first = Xd != nullptr ? 0 : nchunks;   // chunk counter runs over [first, 2 nchunks)
-  const int total = 2 * nchunks;
-  for (int cc = first; cc < total; ++cc) {
-    const int st = (cc - first) % TC_STAGES;
+  const uint32_t tmem = tc_mainloop(s, tid, row < M, 2 * nchunks - first, [&](int i) {
+    const int cc = first + i;
     const bool tangent_w = cc >= nchunks;          // phase 1: A = X, B = tangent weight images
     const int c = tangent_w ? cc - nchunks : cc;
-    if (cc - first >= TC_STAGES) { mbar_wait(&s.empty[st], ph_empty[st]); ph_empty[st] ^= 1; }
-    if (tid == 0) {
-      mbar_expect_tx(&s.full_b[st], B_BYTES);
-      tma_bulk_g2s(s.b[st], (tangent_w ? tiles_d : tiles) + (int64_t)c * (2 * NT * TC_KC), B_BYTES, &s.full_b[st]);
-    }
-    {
-      float* ahi = s.a[st][0];
-      float* alo = s.a[st][1];
-      const int base = ((tid >> 3) * 8) * 32 + (tid & 7) * 4;
-      const float* xr = (tangent_w ? X : Xd) + row * ldx + c * TC_KC;
-#pragma unroll
-      for (int kc = 0; kc < 8; ++kc) {
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (row < M && c * TC_KC + kc * 4 < Kred) v = *reinterpret_cast<const float4*>(xr + kc * 4);
-        float4 h = make_float4(tf32_hi(v.x), tf32_hi(v.y), tf32_hi(v.z), tf32_hi(v.w));
-        *reinterpret_cast<float4*>(ahi + base + kc * 32) = h;
-        if (PASSES == 3) *reinterpret_cast<float4*>(alo + base + kc * 32) = make_float4(tf32_lo(v.x, h.x), tf32_lo(v.y, h.y), tf32_lo(v.z, h.z), tf32_lo(v.w, h.w));
-      }
-    }
-    fence_async_smem();
-    __syncthreads();
-    if (tid == 0) {
-      mbar_wait(&s.full_b[st], ph_full[st]);
-      tc_fence_after();
-      const uint32_t a_hi = smem_u32(s.a[st][0]), a_lo = smem_u32(s.a[st][1]);
-      const uint32_t b_hi = smem_u32(s.b[st]), b_lo = b_hi + NT * TC_KC * sizeof(float);
-#pragma unroll
-      for (int j = 0; j < TC_KC / 8; ++j) {
-        const uint32_t off = j * 256;
-        const uint64_t dah = umma_desc(a_hi + off, 128, 1024), dbh = umma_desc(b_hi + off, 128, 1024);
-        umma_tf32(tmem, dah, dbh, idesc, ((cc - first) | j) != 0);
-        if (PASSES == 3) {
-          const uint64_t dal = umma_desc(a_lo + off, 128, 1024), dbl = umma_desc(b_lo + off, 128, 1024);
-          umma_tf32(tmem, dal, dbh, idesc, 1);
-          umma_tf32(tmem, dah, dbl, idesc, 1);
-        }
-      }
-      umma_commit(&s.empty[st]);
-      if (cc == total - 1) umma_commit(&s.done);
-    }
-    ph_full[st] ^= 1;
-  }
-  mbar_wait(&s.done, 0);
-  tc_fence_after();
+    return TcChunk{(tangent_w ? X : Xd) + row * ldx + c * TC_KC, Kred - c * TC_KC,
+                   (tangent_w ? tiles_d : tiles) + (int64_t)c * (2 * NT * TC_KC)};
+  });
 
   // ---- epilogue (thread = row): Z tile staged through the idle operand stage, transformed in place into yd
   constexpr int CPR = NT / 4;
@@ -753,7 +569,7 @@ __global__ void __launch_bounds__(128, 1) tc_jvp_linear_ln_kernel(const float* _
   float s1 = 0.f, s2 = 0.f;
   for (int c0 = 0; c0 < Np; c0 += 32) {
     float v[32];
-    tmem_ld32(trow + c0, v);
+    um::tmem_ld32(trow + c0, v);
 #pragma unroll
     for (int j4 = 0; j4 < 32; j4 += 4) {
       if (c0 + j4 < Np) {
@@ -776,7 +592,7 @@ __global__ void __launch_bounds__(128, 1) tc_jvp_linear_ln_kernel(const float* _
   const float m1 = s1 * inv_n, m2 = s2 * inv_n;
   for (int c0 = 0; c0 < Np; c0 += 32) {
     float v[32];
-    tmem_ld32(trow + c0, v);
+    um::tmem_ld32(trow + c0, v);
 #pragma unroll
     for (int j4 = 0; j4 < 32; j4 += 4) {
       if (c0 + j4 < Np) {
@@ -812,12 +628,12 @@ __global__ void __launch_bounds__(128, 1) tc_jvp_linear_ln_kernel(const float* _
         *reinterpret_cast<float4*>(Yd + (row0 + r) * Np + lc * 4) = tile[r * CPR + (lc ^ (r & (CPR - 1) & 31))];
     }
   }
-  tc_fence_before();
+  um::tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)NT) : "memory");
+  if (warp == 0) um::tmem_dealloc(tmem, NT);
 }
 
-template <int NT, int PASSES>
+template <int NT>
 static int launch_tc_jvp_nt(int act, const float* X, int ldx, const float* Xd, const float* tiles, const float* tiles_d,
                             int nchunks, const float* bd, const float* lnw, const float* lnwd, const float* lnbd,
                             const float* Z, const float* stats, float* Yd, int64_t M, int N, int Kred, cudaStream_t st) {
@@ -825,7 +641,7 @@ static int launch_tc_jvp_nt(int act, const float* X, int ldx, const float* Xd, c
   dim3 grid((unsigned)ceil_div64(M, TC_BM));
 #define HB_TC_CASE(A)                                                                                       \
   case A: {                                                                                                 \
-    auto kern = tc_jvp_linear_ln_kernel<NT, A, PASSES>;                                                     \
+    auto kern = tc_jvp_linear_ln_kernel<NT, A>;                                                             \
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                     \
     kern<<<grid, 128, smem, st>>>(X, ldx, Xd, tiles, tiles_d, nchunks, bd, lnw, lnwd, lnbd, Z, stats, Yd, M, N, Kred); \
   } break;
@@ -835,19 +651,18 @@ static int launch_tc_jvp_nt(int act, const float* X, int ldx, const float* Xd, c
     default: set_error("activation %d", act); return HB_ERR_UNSUPPORTED;
   }
 #undef HB_TC_CASE
-  HB_LAUNCH_DONE(st, shape_label(PASSES == 3 ? "tc_jvp_linear_ln_3xtf32" : "tc_jvp_linear_ln_tf32", M, N, Kred));
+  HB_LAUNCH_DONE(st, shape_label("tc_jvp_linear_ln_3xtf32", M, N, Kred));
   return HB_OK;
 }
 
-int launch_tc_jvp_linear_ln(int passes, int act, const float* X, int ldx, const float* Xd, const float* tiles,
+int launch_tc_jvp_linear_ln(int act, const float* X, int ldx, const float* Xd, const float* tiles,
                             const float* tiles_d, int nchunks, const float* bd, const float* lnw, const float* lnwd,
                             const float* lnbd, const float* Z, const float* stats, float* Yd, int64_t M, int N, int Kred,
                             cudaStream_t st) {
   if (M <= 0) return HB_OK;
 #define HB_TC_NT(NTV)                                                                                                   \
   case NTV:                                                                                                             \
-    return passes == 3 ? launch_tc_jvp_nt<NTV, 3>(act, X, ldx, Xd, tiles, tiles_d, nchunks, bd, lnw, lnwd, lnbd, Z, stats, Yd, M, N, Kred, st) \
-                       : launch_tc_jvp_nt<NTV, 1>(act, X, ldx, Xd, tiles, tiles_d, nchunks, bd, lnw, lnwd, lnbd, Z, stats, Yd, M, N, Kred, st);
+    return launch_tc_jvp_nt<NTV>(act, X, ldx, Xd, tiles, tiles_d, nchunks, bd, lnw, lnwd, lnbd, Z, stats, Yd, M, N, Kred, st);
   switch (tc_nt_of(N)) { HB_TC_NT(32) HB_TC_NT(64) HB_TC_NT(128) HB_TC_NT(256) }
 #undef HB_TC_NT
   return HB_ERR_UNSUPPORTED;
@@ -868,7 +683,7 @@ struct TcDwSmem {
   uint32_t tmem_base;
 };
 
-template <int NTK, int PASSES>
+template <int NTK>
 __global__ void __launch_bounds__(128, 1) tc_dw_accum_kernel(const float* __restrict__ dZ, int N,
                                                              const float* __restrict__ X, int ldx, int K,
                                                              float* __restrict__ dW, float* __restrict__ db, int64_t M,
@@ -881,19 +696,16 @@ __global__ void __launch_bounds__(128, 1) tc_dw_accum_kernel(const float* __rest
   const int64_t m0 = (int64_t)blockIdx.x * rows_per_cta;
   const int64_t m1 = m0 + rows_per_cta < M ? m0 + rows_per_cta : M;
   if (tid == 0) {
-    for (int i = 0; i < TC_STAGES; ++i) mbar_init(&s.empty[i], 1);
-    mbar_init(&s.done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int i = 0; i < TC_STAGES; ++i) um::mbar_init(&s.empty[i], 1);
+    um::mbar_init(&s.done, 1);
+    um::fence_mbarrier_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s.tmem_base)), "r"((uint32_t)NTK) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
+  if (warp == 0) um::tmem_alloc(&s.tmem_base, NTK);
+  um::tc_fence_before();
   __syncthreads();
-  tc_fence_after();
+  um::tc_fence_after();
   const uint32_t tmem = s.tmem_base;
-  constexpr uint32_t idesc = umma_idesc_tf32(NTK);
+  constexpr uint32_t idesc = um::idesc_tf32(NTK);
   const int nchunks = (int)((m1 - m0 + TC_KC - 1) / TC_KC);
   uint32_t ph_empty[2] = {0, 0};
   float bsum = 0.f;
@@ -924,14 +736,14 @@ __global__ void __launch_bounds__(128, 1) tc_dw_accum_kernel(const float* __rest
   if (nchunks > 0) load_chunk(0);
   for (int c = 0; c < nchunks; ++c) {
     const int st = c % TC_STAGES;
-    if (c >= TC_STAGES) { mbar_wait(&s.empty[st], ph_empty[st]); ph_empty[st] ^= 1; }
+    if (c >= TC_STAGES) { um::mbar_wait(&s.empty[st], ph_empty[st]); ph_empty[st] ^= 1; }
 #pragma unroll
     for (int kc = 0; kc < 8; ++kc) {
       const float* v = va + kc * 4;
       bsum += (v[0] + v[1]) + (v[2] + v[3]);
       const float4 h = make_float4(tf32_hi(v[0]), tf32_hi(v[1]), tf32_hi(v[2]), tf32_hi(v[3]));
       *reinterpret_cast<float4*>(&s.a[st][0][slot + kc * 32]) = h;
-      if (PASSES == 3) *reinterpret_cast<float4*>(&s.a[st][1][slot + kc * 32]) = make_float4(tf32_lo(v[0], h.x), tf32_lo(v[1], h.y), tf32_lo(v[2], h.z), tf32_lo(v[3], h.w));
+      *reinterpret_cast<float4*>(&s.a[st][1][slot + kc * 32]) = make_float4(tf32_lo(v[0], h.x), tf32_lo(v[1], h.y), tf32_lo(v[2], h.z), tf32_lo(v[3], h.w));
     }
 #pragma unroll
     for (int fb = 0; fb < NB; ++fb) {
@@ -943,42 +755,40 @@ __global__ void __launch_bounds__(128, 1) tc_dw_accum_kernel(const float* __rest
           const float* v = vb[fb] + kc * 4;
           const float4 h = make_float4(tf32_hi(v[0]), tf32_hi(v[1]), tf32_hi(v[2]), tf32_hi(v[3]));
           *reinterpret_cast<float4*>(&s.b[st][0][bslot + kc * 32]) = h;
-          if (PASSES == 3) *reinterpret_cast<float4*>(&s.b[st][1][bslot + kc * 32]) = make_float4(tf32_lo(v[0], h.x), tf32_lo(v[1], h.y), tf32_lo(v[2], h.z), tf32_lo(v[3], h.w));
+          *reinterpret_cast<float4*>(&s.b[st][1][bslot + kc * 32]) = make_float4(tf32_lo(v[0], h.x), tf32_lo(v[1], h.y), tf32_lo(v[2], h.z), tf32_lo(v[3], h.w));
         }
       }
     }
     if (c + 1 < nchunks) load_chunk(c + 1);
-    fence_async_smem();
+    um::fence_async_smem();
     __syncthreads();
     if (tid == 0) {
-      tc_fence_after();
-      const uint32_t a_hi = smem_u32(s.a[st][0]), a_lo = smem_u32(s.a[st][1]);
-      const uint32_t b_hi = smem_u32(s.b[st][0]), b_lo = smem_u32(s.b[st][1]);
+      um::tc_fence_after();
+      const uint32_t a_hi = um::smem_u32(s.a[st][0]), a_lo = um::smem_u32(s.a[st][1]);
+      const uint32_t b_hi = um::smem_u32(s.b[st][0]), b_lo = um::smem_u32(s.b[st][1]);
 #pragma unroll
       for (int j = 0; j < TC_KC / 8; ++j) {
         const uint32_t off = j * 256;
-        const uint64_t dah = umma_desc(a_hi + off, 128, 1024), dbh = umma_desc(b_hi + off, 128, 1024);
-        umma_tf32(tmem, dah, dbh, idesc, (c | j) != 0);
-        if (PASSES == 3) {
-          const uint64_t dal = umma_desc(a_lo + off, 128, 1024), dbl = umma_desc(b_lo + off, 128, 1024);
-          umma_tf32(tmem, dal, dbh, idesc, 1);
-          umma_tf32(tmem, dah, dbl, idesc, 1);
-        }
+        const uint64_t dah = um::desc(a_hi + off, 128, 1024), dbh = um::desc(b_hi + off, 128, 1024);
+        um::mma_tf32(tmem, dah, dbh, idesc, (c | j) != 0);
+        const uint64_t dal = um::desc(a_lo + off, 128, 1024), dbl = um::desc(b_lo + off, 128, 1024);
+        um::mma_tf32(tmem, dal, dbh, idesc, 1);
+        um::mma_tf32(tmem, dah, dbl, idesc, 1);
       }
-      umma_commit(&s.empty[st]);
-      if (c == nchunks - 1) umma_commit(&s.done);
+      um::commit(&s.empty[st]);
+      if (c == nchunks - 1) um::commit(&s.done);
     }
   }
   if (nchunks > 0) {
-    mbar_wait(&s.done, 0);
-    tc_fence_after();
+    um::mbar_wait(&s.done, 0);
+    um::tc_fence_after();
     const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
     // part_stride != 0: this CTA owns slot blockIdx.x of a split buffer [splits][params] -> plain read-modify-write
     // (deterministic, no atomics; summed into the gradient once per call by dw_reduce_kernel).  Else: atomics into dW.
     float* dst = dW + (int64_t)blockIdx.x * part_stride + (int64_t)fa * K;
     for (int c0 = 0; c0 < NTK && k0 + c0 < K; c0 += 32) {
       float v[32];
-      tmem_ld32(trow + c0, v);
+      um::tmem_ld32(trow + c0, v);
       if (fa < N) {
         if (part_stride != 0 && (K & 3) == 0) {
 #pragma unroll
@@ -1003,9 +813,9 @@ __global__ void __launch_bounds__(128, 1) tc_dw_accum_kernel(const float* __rest
     }
     if (db != nullptr && fa < N && blockIdx.z == 0) atomicAdd(db + fa, bsum);
   }
-  tc_fence_before();
+  um::tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)NTK) : "memory");
+  if (warp == 0) um::tmem_dealloc(tmem, NTK);
 }
 
 constexpr int TC_DW_SPLITS = tc_dw_splits_c();
@@ -1028,7 +838,7 @@ int launch_dw_reduce(float* grad, const float* part, int total, cudaStream_t st)
 }
 
 template <int NTK>
-static int launch_tc_dw_ntk(int passes, const float* dZ, int N, const float* X, int ldx, int K, float* dW, float* db,
+static int launch_tc_dw_ntk(const float* dZ, int N, const float* X, int ldx, int K, float* dW, float* db,
                             int64_t M, int64_t part_stride, cudaStream_t st) {
   const int nb = (N + 127) / 128, kb = (ldx + NTK - 1) / NTK;
   int64_t splits, rows_per;
@@ -1043,27 +853,21 @@ static int launch_tc_dw_ntk(int passes, const float* dZ, int N, const float* X, 
   }
   const size_t smem = sizeof(TcDwSmem<NTK>) + 1024;
   dim3 grid((unsigned)splits, nb, kb);
-  if (passes == 3) {
-    auto kern = tc_dw_accum_kernel<NTK, 3>;
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kern<<<grid, 128, smem, st>>>(dZ, N, X, ldx, K, dW, db, M, rows_per, part_stride);
-  } else {
-    auto kern = tc_dw_accum_kernel<NTK, 1>;
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kern<<<grid, 128, smem, st>>>(dZ, N, X, ldx, K, dW, db, M, rows_per, part_stride);
-  }
-  HB_LAUNCH_DONE(st, shape_label(passes == 3 ? "tc_dw_accum_3xtf32" : "tc_dw_accum_tf32", M, N, K));
+  auto kern = tc_dw_accum_kernel<NTK>;
+  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  kern<<<grid, 128, smem, st>>>(dZ, N, X, ldx, K, dW, db, M, rows_per, part_stride);
+  HB_LAUNCH_DONE(st, shape_label("tc_dw_accum_3xtf32", M, N, K));
   return HB_OK;
 }
 
-int launch_tc_dw_accum(int passes, const float* dZ, int N, const float* X, int ldx, int K, float* dW, float* db,
+int launch_tc_dw_accum(const float* dZ, int N, const float* X, int ldx, int K, float* dW, float* db,
                        int64_t M, int64_t part_stride, cudaStream_t st) {
   if (M <= 0) return HB_OK;
   switch (tc_nt_of(ldx)) {
-    case 32: return launch_tc_dw_ntk<32>(passes, dZ, N, X, ldx, K, dW, db, M, part_stride, st);
-    case 64: return launch_tc_dw_ntk<64>(passes, dZ, N, X, ldx, K, dW, db, M, part_stride, st);
-    case 128: return launch_tc_dw_ntk<128>(passes, dZ, N, X, ldx, K, dW, db, M, part_stride, st);
-    default: return launch_tc_dw_ntk<256>(passes, dZ, N, X, ldx, K, dW, db, M, part_stride, st);
+    case 32: return launch_tc_dw_ntk<32>(dZ, N, X, ldx, K, dW, db, M, part_stride, st);
+    case 64: return launch_tc_dw_ntk<64>(dZ, N, X, ldx, K, dW, db, M, part_stride, st);
+    case 128: return launch_tc_dw_ntk<128>(dZ, N, X, ldx, K, dW, db, M, part_stride, st);
+    default: return launch_tc_dw_ntk<256>(dZ, N, X, ldx, K, dW, db, M, part_stride, st);
   }
 }
 

@@ -1,5 +1,7 @@
-// tcgen05 / TMA / mbarrier inline-PTX helpers for the fused update kernel (fused_update.cu), sm_100a only.
-// Operand layouts: canonical no-swizzle core matrices of 8 rows x 16 bytes.  A ROW-WRITTEN tile
+// tcgen05 / TMA / mbarrier inline-PTX helpers for every tensor-core kernel (fused_update.cu, tc_gemm.cu), sm_100a only.
+// Two MMA kinds: kind::f16 (fp16 operands, the fused update kernel) and kind::tf32 (fp32 operands read as TF32, the
+// layer-wise kernels); both accumulate fp32 in TMEM with M = 128.
+// fp16 operand layouts: canonical no-swizzle core matrices of 8 rows x 16 bytes.  A ROW-WRITTEN tile
 //     IMG[row/8][chunk][row%8][16 B]      (chunk = 8 fp16 features)
 // serves as a K-major operand (M/N index = row, K = feature: LBO = 128 B between the two k-chunks of an MMA, SBO = bytes
 // between 8-row groups) AND as an MN-major operand (M/N index = feature, K = row: SBO = 128 B between feature chunks,
@@ -16,6 +18,8 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
 }
+// after the mbarrier.init's of a CTA, before the barrier that publishes them
+__device__ __forceinline__ void fence_mbarrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
@@ -40,6 +44,16 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
+// TMEM allocation, by one whole warp: `cols` columns (a power of two >= 32), base address written to *slot; the permit is
+// relinquished at once so that other CTAs on the SM can allocate.  The same warp frees them with tmem_dealloc.
+__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t cols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols) : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+}
+
 // shared-memory matrix descriptor, SWIZZLE_NONE, version 1 (cute::UMMA::SmemDescriptor bit layout)
 __device__ __forceinline__ uint64_t desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = (uint64_t)((saddr & 0x3FFFFu) >> 4);
@@ -57,6 +71,17 @@ __device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+// instruction descriptor: D fp32, A/B tf32, both K-major, M = 128, N = n
+__host__ __device__ constexpr uint32_t idesc_tf32(int n) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+}
+__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
 __device__ __forceinline__ void commit(uint64_t* bar) {

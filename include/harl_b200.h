@@ -100,7 +100,7 @@ int hb_profile_begin(void* stream);
 int hb_profile_end(char* out, int out_size);
 
 /* GEMM implementation of the MLP blocks: 0 = FP32 SIMT, 1 = tcgen05 tensor cores with the error-compensated
- * 3xTF32 split (fp32-level accuracy; default), 2 = tcgen05 plain TF32.  Call hb_net_prepare after
+ * 3xTF32 split (fp32-level accuracy; default); any other value returns HB_ERR_INVALID.  Call hb_net_prepare after
  * changing it (the tensor-core path reads pre-packed operand images from the prepared buffer). */
 int hb_set_gemm_impl(int impl);
 int hb_get_gemm_impl(void);
@@ -234,10 +234,11 @@ int hb_allreduce_bucket(void* comm, void* buf, int64_t n, int32_t dtype, void* s
 int hb_comm_status(void* comm);
 int hb_comm_destroy(void* comm);
 
-/* Which kernel runs the GAE branch of hb_gae_returns: 0 = column tiles staged in shared memory (gae.cu),
- * 1 = time-segmented, register-resident, sequential carry (default; bit-identical to 0 and to the reference's
- * on_policy_critic_buffer_ep.py:111-140 loop), 2 = same with a parallel affine scan for the carry between segments
- * (advantages within 1e-6 of max|adv| of the sequential result).  Env HB_GAE_IMPL sets the initial value. */
+/* How the time-segmented GAE kernel (T <= 256) carries the running GAE between its segments: 1 = sequentially
+ * (default; bit-identical to the reference's on_policy_critic_buffer_ep.py:111-140 loop), 2 = by a parallel affine scan
+ * (advantages within 1e-6 of max|adv| of the sequential result); any other value returns HB_ERR_INVALID.  Longer
+ * rollouts and the return branch without GAE always run the bit-exact column-tile kernel.  Env HB_GAE_IMPL=2 selects 2
+ * at start-up; any other value gives 1. */
 int hb_set_gae_impl(int impl);
 int hb_get_gae_impl(void);
 

@@ -19,11 +19,8 @@ print(json.dumps(out))
 """ % ROOT
 
 print("# variant                          [200,4096] us  GB/s  copy us | [200,65536] us  GB/s  copy us")
-for name, env in (("tiled cp.async (round 1)", dict(HB_GAE_IMPL="0")),
-                  ("segmented exact, 8 x 25", dict(HB_GAE_IMPL="1")),
-                  ("segmented exact, 13 x 16", dict(HB_GAE_IMPL="1", HB_GAE_SEGS="13")),
-                  ("segmented scan, 8 x 25", dict(HB_GAE_IMPL="2")),
-                  ("segmented scan, 13 x 16", dict(HB_GAE_IMPL="2", HB_GAE_SEGS="13"))):
+for name, env in (("segmented, sequential carry", dict(HB_GAE_IMPL="1")),
+                  ("segmented, parallel-scan carry", dict(HB_GAE_IMPL="2"))):
     r = subprocess.run([sys.executable, "-c", CODE], env={**os.environ, **env}, capture_output=True, text=True)
     if r.returncode != 0:
         print(name, "FAILED", r.stderr[-500:])

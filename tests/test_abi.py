@@ -121,6 +121,16 @@ def test_workspace_sizing_and_argument_checks(L):
     assert rc == -1 and b"NULL" in L.lib.hb_last_error()
 
 
+def test_impl_setters_reject_unknown_values(L):
+    """hb_set_gemm_impl takes 0 / 1 and hb_set_gae_impl 1 / 2: any other value is refused and changes nothing."""
+    gemm, gae = L.lib.hb_get_gemm_impl(), L.lib.hb_get_gae_impl()
+    for setter, bad in (("hb_set_gemm_impl", 2), ("hb_set_gae_impl", 0), ("hb_set_gae_impl", 3)):
+        assert getattr(L.lib, setter)(bad) == -1 and b"impl must be" in L.lib.hb_last_error()
+        assert (L.lib.hb_get_gemm_impl(), L.lib.hb_get_gae_impl()) == (gemm, gae)
+    assert L.lib.hb_set_gae_impl(2) == 0 and L.lib.hb_get_gae_impl() == 2
+    assert L.lib.hb_set_gae_impl(gae) == 0 and L.lib.hb_get_gae_impl() == gae
+
+
 def test_recurrent_and_trust_region_workspace_sizing(L):
     """Host-only sizing calls: recurrent batches are never chunked (a chunk would cut every sequence), so their
     workspace keeps growing with the row count; the trust-region workspace covers the gradient workspace plus the
